@@ -54,7 +54,14 @@ def parse_args():
     ap.add_argument("--no-fusion", action="store_true", help="one kernel sweep per gate")
     ap.add_argument("--no-extras", action="store_true", help="skip the unfused / per-kernel / CPU side measurements")
     ap.add_argument("--cpu-seconds", type=float, default=20.0, help="budget of the cpu_baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the state the last timed step computed (a fixed seeded sample of it) to DIR as .npy files")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times a sample of the gates, not whole steps")
+    return args
 
 
 def ncu_traffic(kernel, algorithmic_bytes):
@@ -126,6 +133,39 @@ class ClockSampler:
         busy = sorted(sm)[len(sm) // 4:] if sm else []  # drop the idle tail of the samples
         return {"sm_mhz": (float(np.median(busy)) if busy else None), "sm_max_mhz": mx,
                 "samples": len(sm), "reasons": sorted(reasons)}
+
+
+# --dump-outputs: at most 2^21 amplitudes with their indices (48 MB in f64), at the same seeded indices in every run
+DUMP_AMPS = 1 << 21
+DUMP_SEED = 0x5EED00D0
+DUMP_CHUNK = 1 << 24
+
+
+def dump_outputs(st, out_dir, rank, world):
+    """Write what a step hands its caller, the 2^n amplitudes of the state, as state_indices.npy (float64 global
+    indices, ascending) and state_amplitudes.npy ([re, im] rows in the state's precision): every amplitude when
+    2^n <= DUMP_AMPS, else the amplitudes at a fixed seeded sample of indices.  Collective over the ranks."""
+    import torch.distributed as dist
+    if st.n < DUMP_AMPS.bit_length():
+        idx = np.arange(1 << st.n, dtype=np.int64)
+    else:
+        idx = np.unique(np.random.default_rng(DUMP_SEED).integers(0, 1 << st.n, size=DUMP_AMPS, dtype=np.int64))
+    lo = rank * st.local_len
+    mine = idx[(idx >= lo) & (idx < lo + st.local_len)] - lo
+    amps = np.empty(mine.size, dtype=st.dtype)
+    buf = np.empty(min(DUMP_CHUNK, st.local_len), dtype=st.dtype)
+    for off in range(0, st.local_len, buf.size):
+        a, b = np.searchsorted(mine, [off, off + buf.size])
+        st.download(buf, offset=off)
+        amps[a:b] = buf[mine[a:b] - off]
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, amps)
+        amps = np.concatenate(parts)
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "state_indices.npy"), idx.astype(np.float64))
+        np.save(os.path.join(out_dir, "state_amplitudes.npy"), amps.view(amps.real.dtype).reshape(-1, 2))
 
 
 def build_workload(args, world):
@@ -378,6 +418,8 @@ def run_b200(args):
     exchanges = (s1["exchanges"] - s0["exchanges"]) / args.steps
     fused_gates = (s1["fused_gates"] - s0["fused_gates"]) / args.steps
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(st, args.dump_outputs, rank, world)
     ms_per_step = ms / args.steps
     gates_total = len(ops)
     gps = gates_total / (ms_per_step / 1e3)
