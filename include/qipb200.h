@@ -207,6 +207,12 @@ int qipb200_state_measure_prob(qipb200_state *state, uint64_t measured, const ui
  * supplied by the caller (the reference calls rand::random). */
 int qipb200_state_soft_measure(qipb200_state *state, const uint64_t *indices, uint32_t n_indices,
                                double r, uint64_t *measured);
+/* K draws at once from the state, without changing it: out[j] is what qipb200_state_soft_measure(state, indices,
+ * n_indices, r[j], &m) returns for the same state (measurement_ops.rs:153-176 applied K times).  r and out are HOST
+ * arrays of n_draws entries; r[j] in [0, 1].  Cost: about one read sweep of the state plus O(n_draws) small gathers,
+ * independent of the qubits measured (all n qubits allowed).  COLLECTIVE on a sharded state: every rank passes the
+ * same indices and draws and receives the same out[]. */
+int qipb200_state_sample(qipb200_state *state, const uint64_t *indices, uint32_t n_indices, const double *r, uint64_t n_draws, uint64_t *out);
 /* measure_state (measurement_ops.rs:220-269): zero the amplitudes that
  * contradict `measured`, scale the rest by 1/sqrt(measured_prob); in place. */
 int qipb200_state_collapse(qipb200_state *state, const uint64_t *indices, uint32_t n_indices,

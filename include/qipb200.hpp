@@ -221,6 +221,12 @@ class B200State {
     ctx_.check(qipb200_state_soft_measure(st_, indices.data(), (uint32_t)indices.size(), r, &m));
     return m;
   }
+  // soft_measure for every draw in `draws`, from one read of the state (qipb200_state_sample); the state is unchanged
+  std::vector<uint64_t> sample(const std::vector<uint64_t> &indices, const std::vector<double> &draws) {
+    std::vector<uint64_t> out(draws.size());
+    ctx_.check(qipb200_state_sample(st_, indices.data(), (uint32_t)indices.size(), draws.data(), draws.size(), out.data()));
+    return out;
+  }
   void collapse(const std::vector<uint64_t> &indices, uint64_t measured, double prob) {  // measure_state, :220-269
     ctx_.check(qipb200_state_collapse(st_, indices.data(), (uint32_t)indices.size(), measured, prob));
   }

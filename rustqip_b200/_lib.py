@@ -28,7 +28,7 @@ EXPORTS = [
     "qipb200_state_set_basis", "qipb200_state_upload", "qipb200_state_download",
     "qipb200_state_apply_op", "qipb200_state_apply_schedule", "qipb200_state_norm2",
     "qipb200_state_sync", "qipb200_state_max_abs_diff", "qipb200_calculate_state", "qipb200_state_measure_probs",
-    "qipb200_state_measure_prob", "qipb200_state_soft_measure", "qipb200_state_collapse",
+    "qipb200_state_measure_prob", "qipb200_state_soft_measure", "qipb200_state_sample", "qipb200_state_collapse",
     "qipb200_state_new_sharded", "qipb200_state_ipc_export", "qipb200_state_ipc_import",
     "qipb200_state_qubit_map", "qipb200_state_exchange_bytes", "qipb200_plan_exchanges",
     "qipb200_state_save", "qipb200_state_load", "qipb200_schedule_parse", "qipb200_schedule_ops", "qipb200_schedule_free", "qipb200_schedule_serialise",
@@ -87,6 +87,8 @@ def lib():
     L.qipb200_state_measure_prob.argtypes = [vp, u64, vp, u32, C.POINTER(C.c_double)]
     L.qipb200_state_soft_measure.restype = i32
     L.qipb200_state_soft_measure.argtypes = [vp, vp, u32, C.c_double, C.POINTER(u64)]
+    L.qipb200_state_sample.restype = i32
+    L.qipb200_state_sample.argtypes = [vp, vp, u32, vp, u64, vp]
     L.qipb200_state_collapse.restype = i32
     L.qipb200_state_collapse.argtypes = [vp, vp, u32, u64, C.c_double]
     L.qipb200_state_new_sharded.restype = i32

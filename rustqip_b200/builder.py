@@ -225,6 +225,23 @@ class B200Builder:
             return st.download(), measurements
 
 
+    def sample_with_init(self, init: Sequence[Tuple[Register, int]], indices, shots: int, rng=None, ctx=None,
+                         fusion: bool = True) -> np.ndarray:
+        """Run the unitary pipeline once from the initial registers and draw `shots` outcomes of the qubits
+        `indices` (a Register or qubit indices; bit i of an outcome from the i-th qubit) from the final state
+        (soft_measure, measurement_ops.rs:153-176, once per shot).  `rng`: a numpy Generator for the draws.
+        A pipeline with a measurement entry is refused: shots after a mid-circuit collapse are not independent."""
+        from .state import State
+        if any(kind == "MEASURE" for _, kind, _ in self.pipeline):
+            raise CircuitError("sample_with_init: the pipeline contains a measurement; shots need a unitary pipeline")
+        qubits = indices.indices if isinstance(indices, Register) else list(indices)
+        draws = (rng if rng is not None else np.random.default_rng()).random(int(shots))
+        with State(self._n, self.dtype, ctx) as st:
+            st.set_basis(self.initial_index(init))
+            st.apply_schedule(self.unitary_ops(), fusion=fusion)
+            return st.sample(qubits, draws)
+
+
 class Conditioned:
     """conditioning.rs:29-85 restricted to what LocalBuilder can decompose without ancillas."""
 

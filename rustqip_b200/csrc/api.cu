@@ -1476,113 +1476,57 @@ int measure_probs_impl(qipb200_state *s, const uint64_t *indices, uint32_t n_ind
   return st;
 }
 
-// The serial scan of measurement_ops.rs:166-172 over this rank's amplitudes, starting with `rem` left of the
-// draw: per-chunk sums on the device, chunk search on the host, then a scan of the chunk holding the crossing
-// (and of the following ones when rounding leaves the chunk-level search one step short).
-int local_scan(qipb200_state *s, double rem, bool *crossed, uint64_t *idx_out) {
-  qipb200_ctx *ctx = s->ctx;
-  const uint64_t len = 1ull << s->n_local;
-  const uint32_t chunk_log2 = s->n_local > 12 ? 12 : s->n_local;
-  const uint64_t chunks = len >> chunk_log2;
-  double *d_sums = nullptr;
-  CU(ctx, cudaMallocAsync((void **)&d_sums, chunks * sizeof(double), ctx->stream));
-  CU(ctx, launch_chunk_sums(s->prec, s->buf, len, chunk_log2, d_sums, ctx->stream, &ctx->launches));
-  std::vector<double> sums(chunks);
-  CU(ctx, cudaMemcpyAsync(sums.data(), d_sums, chunks * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-  CU(ctx, cudaFreeAsync(d_sums, ctx->stream));
-  CU(ctx, cudaStreamSynchronize(ctx->stream));
-  uint64_t c = 0;
-  for (; c + 1 < chunks; ++c) {
-    if (rem - sums[c] <= 0.0) break;
-    rem -= sums[c];
-  }
-  const uint64_t clen = 1ull << chunk_log2;
-  const size_t ab = amp_bytes(s->prec);
-  std::vector<char> host(clen * ab);
-  *crossed = false;
-  *idx_out = 0;
-  for (; c < chunks && !*crossed; ++c) {
-    CU(ctx, cudaMemcpyAsync(host.data(), (const char *)s->buf + c * clen * ab, clen * ab, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream));
-    for (uint64_t i = 0; i < clen; ++i) {
-      double re, im;
-      if (s->prec == QIP_F32) {
-        re = ((const float *)host.data())[2 * i];
-        im = ((const float *)host.data())[2 * i + 1];
-      } else {
-        re = ((const double *)host.data())[2 * i];
-        im = ((const double *)host.data())[2 * i + 1];
-      }
-      rem -= re * re + im * im;
-      if (rem <= 0.0) {
-        *idx_out = c * clen + i;
-        *crossed = true;
-        break;
-      }
-    }
-  }
-  return QIPB200_OK;
-}
-
-int soft_measure_impl(qipb200_state *s, const uint64_t *indices, uint32_t n_indices, double r, uint64_t *measured) {
+// Inverse-CDF sampling of n_draws draws (measurement_ops.rs:153-176 applied to each; rules in sample.cuh): one read
+// sweep for the chunk sums, their prefix, then one warp per draw.  The reference scans in canonical index order, so a
+// permuted layout is restored first (collective on a sharded state: rank t then holds [t 2^nl, (t+1) 2^nl)).  The
+// ranks' totals are all-reduced, the owner of each draw resolves it, and the indices are summed across the ranks.
+int sample_impl(qipb200_state *s, const uint64_t *indices, uint32_t n_indices, const double *r, uint64_t n_draws,
+                uint64_t *out) {
   qipb200_ctx *ctx = s->ctx;
   CU(ctx, cudaSetDevice(ctx->device));
-  uint64_t idx = 0;  // the reference leaves measured_indx = 0 when the scan never crosses
-  if (s->world == 1) {
-    bool crossed = false;
-    int st = local_scan(s, r, &crossed, &idx);  // full-length input: r * 1 (measurement_ops.rs:160-165)
-    if (st != QIPB200_OK) return st;
-  } else {
-    // The reference scans the whole vector in index order: restore the canonical layout (rank r then holds
-    // indices [r 2^nl, (r+1) 2^nl)), all-gather the per-rank totals, let every rank scan its own shard with the
-    // part of the draw the lower ranks left over, all-gather (crossed, index): the lowest crossing rank wins.
-    if (!layout_is_identity(s)) {
-      int st = restore_layout(s);
-      if (st != QIPB200_OK) return st;
-    }
-    const int W = s->world;
-    double *d_vec = nullptr;
-    CU(ctx, cudaMallocAsync((void **)&d_vec, 2 * W * sizeof(double), ctx->stream));
-    CU(ctx, cudaMemsetAsync(d_vec, 0, 2 * W * sizeof(double), ctx->stream));
-    CU(ctx, launch_norm2(s->prec, s->buf, 1ull << s->n_local, ctx->d_scalar, ctx->stream, &ctx->launches));
-    CU(ctx, cudaMemcpyAsync(d_vec + s->rank, ctx->d_scalar, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-    int st = allreduce_sum(s, d_vec, (uint32_t)W);
-    std::vector<double> tot(2 * W, 0.0);
-    if (st == QIPB200_OK) {
-      CU(ctx, cudaMemcpyAsync(tot.data(), d_vec, W * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-      CU(ctx, cudaStreamSynchronize(ctx->stream));
-      double rem = r;
-      for (int t = 0; t < s->rank; ++t) rem -= tot[t];
-      bool crossed = false;
-      uint64_t li = 0;
-      if (rem <= 0.0 && s->rank > 0) {
-        crossed = true;  // the draw ran out below this rank: a serial scan arriving here stops at the first element
-      } else {
-        st = local_scan(s, rem, &crossed, &li);
-      }
-      std::vector<double> mine(2 * W, 0.0);
-      mine[2 * s->rank] = crossed ? 1.0 : 0.0;
-      mine[2 * s->rank + 1] = (double)(((uint64_t)s->rank << s->n_local) + li);  // < 2^40: exact in a double
-      if (st == QIPB200_OK) {
-        CU(ctx, cudaMemcpyAsync(d_vec, mine.data(), 2 * W * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-        st = allreduce_sum(s, d_vec, (uint32_t)(2 * W));
-      }
-      if (st == QIPB200_OK) {
-        CU(ctx, cudaMemcpyAsync(tot.data(), d_vec, 2 * W * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        CU(ctx, cudaStreamSynchronize(ctx->stream));
-        for (int t = 0; t < W; ++t)
-          if (tot[2 * t] != 0.0) {
-            idx = (uint64_t)tot[2 * t + 1];
-            break;
-          }
-      }
-    }
-    CU(ctx, cudaFreeAsync(d_vec, ctx->stream));
+  if (!layout_is_identity(s)) {
+    int st = restore_layout(s);
     if (st != QIPB200_OK) return st;
   }
-  uint64_t m = 0;  // extract_bits(measured_indx, [n-1-index]) (measurement_ops.rs:174-175)
-  for (uint32_t i = 0; i < n_indices; ++i) m |= ((idx >> (s->n - 1 - indices[i])) & 1ull) << i;
-  *measured = m;
+  const int W = s->world;
+  SampleArgs a;
+  a.n_draws = 0;
+  a.chunk_log2 = std::min<uint32_t>(s->n_local, kSampleChunkLog2);
+  a.chunks = 1ull << (s->n_local - a.chunk_log2);
+  a.index_base = (uint64_t)s->rank << s->n_local;
+  a.rank = s->rank;
+  a.world = W;
+  uint8_t bitpos[64];
+  for (uint32_t i = 0; i < n_indices; ++i) bitpos[i] = (uint8_t)(s->n - 1 - indices[i]);
+  const uint64_t batch = std::min<uint64_t>(n_draws, kSampleBatch);
+  // [chunk prefix | rank totals | draws | results]
+  double *d_P = nullptr;
+  CU(ctx, cudaMallocAsync((void **)&d_P, (a.chunks + W + 2 * batch) * sizeof(double), ctx->stream));
+  double *d_tot = d_P + a.chunks, *d_draw = d_tot + W, *d_res = d_draw + batch;
+  auto run = [&]() -> int {
+    CU(ctx, launch_chunk_sums(s->prec, s->buf, 1ull << s->n_local, a.chunk_log2, d_P, ctx->stream, &ctx->launches));
+    CU(ctx, launch_sample_scan(d_P, a.chunks, ctx->stream, &ctx->launches));
+    // a rank's total is the last prefix: the owner's chunk search always finds the chunk its share of the draw is in
+    CU(ctx, cudaMemsetAsync(d_tot, 0, W * sizeof(double), ctx->stream));
+    CU(ctx, cudaMemcpyAsync(d_tot + s->rank, d_P + a.chunks - 1, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+    int st = allreduce_sum(s, d_tot, (uint32_t)W);
+    for (uint64_t done = 0; st == QIPB200_OK && done < n_draws; done += a.n_draws) {
+      a.n_draws = std::min<uint64_t>(batch, n_draws - done);
+      CU(ctx, cudaMemcpyAsync(d_draw, r + done, a.n_draws * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+      CU(ctx, launch_sample_resolve(s->prec, s->buf, d_P, d_tot, d_draw, d_res, a, ctx->stream, &ctx->launches));
+      for (uint64_t o = 0; st == QIPB200_OK && W > 1 && o < a.n_draws; o += (uint64_t)kCommDoubles)
+        st = allreduce_sum(s, d_res + o, (uint32_t)std::min<uint64_t>((uint64_t)kCommDoubles, a.n_draws - o));
+      if (st != QIPB200_OK) break;
+      CU(ctx, launch_sample_outcomes(d_res, a.n_draws, bitpos, n_indices, ctx->stream, &ctx->launches));
+      CU(ctx, cudaMemcpyAsync(out + done, d_res, a.n_draws * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    return st;
+  };
+  int st = run();
+  cudaFreeAsync(d_P, ctx->stream);
+  if (st != QIPB200_OK) return st;
+  CU(ctx, cudaStreamSynchronize(ctx->stream));
+  if (W > 1) return check_barrier_error(s);
   return QIPB200_OK;
 }
 
@@ -1640,19 +1584,46 @@ extern "C" int qipb200_state_measure_prob(qipb200_state *s, uint64_t measured, c
   });
 }
 
+// Every rank of a multi-device state computes the same answers; rank 0's are returned after the others are compared.
+static int multi_sample(qipb200_state *s, const uint64_t *indices, uint32_t n_indices, const double *r, uint64_t n_draws,
+                        uint64_t *out) {
+  const size_t G = s->shards.size();
+  std::vector<std::vector<uint64_t>> v(G);
+  for (size_t k = 1; k < G; ++k) v[k].resize(n_draws);
+  int st = each_shard(s, [&](qipb200_state *sh, int rk) {
+    return sample_impl(sh, indices, n_indices, r, n_draws, rk == 0 ? out : v[rk].data());
+  });
+  if (st != QIPB200_OK) return st;
+  for (size_t k = 1; k < G; ++k)
+    if (n_draws && memcmp(v[k].data(), out, n_draws * sizeof(uint64_t)) != 0)
+      return set_err(s->ctx, QIPB200_ERR_COMM, "sample: the shards disagree on the drawn outcomes");
+  return QIPB200_OK;
+}
+
 extern "C" int qipb200_state_soft_measure(qipb200_state *s, const uint64_t *indices, uint32_t n_indices, double r,
                                           uint64_t *measured) {
   if (!s || !measured) return set_err(s ? s->ctx : nullptr, QIPB200_ERR_INVALID_ARG, "soft_measure: NULL argument");
   return guarded(s->ctx, [&]() -> int {
     int st = check_indices(s, indices, n_indices);
     if (st != QIPB200_OK) return st;
-    if (!s->shards.empty()) {
-      std::vector<uint64_t> v(s->shards.size(), 0);
-      st = each_shard(s, [&](qipb200_state *sh, int rk) { return soft_measure_impl(sh, indices, n_indices, r, &v[rk]); });
-      *measured = v[0];
-      return st;
-    }
-    return soft_measure_impl(s, indices, n_indices, r, measured);
+    if (!s->shards.empty()) return multi_sample(s, indices, n_indices, &r, 1, measured);
+    return sample_impl(s, indices, n_indices, &r, 1, measured);
+  });
+}
+
+extern "C" int qipb200_state_sample(qipb200_state *s, const uint64_t *indices, uint32_t n_indices, const double *r,
+                                    uint64_t n_draws, uint64_t *out) {
+  if (!s || !r || !out)
+    return set_err(s ? s->ctx : nullptr, QIPB200_ERR_INVALID_ARG, "sample: NULL argument");
+  return guarded(s->ctx, [&]() -> int {
+    int st = check_indices(s, indices, n_indices);
+    if (st != QIPB200_OK) return st;
+    for (uint64_t j = 0; j < n_draws; ++j)
+      if (!(r[j] >= 0.0 && r[j] <= 1.0))
+        return set_err(s->ctx, QIPB200_ERR_INVALID_ARG, "sample: draw " + std::to_string(j) + " is not in [0, 1]");
+    if (n_draws == 0) return (int)QIPB200_OK;
+    if (!s->shards.empty()) return multi_sample(s, indices, n_indices, r, n_draws, out);
+    return sample_impl(s, indices, n_indices, r, n_draws, out);
   });
 }
 

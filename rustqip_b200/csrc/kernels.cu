@@ -1268,6 +1268,146 @@ cudaError_t launch_chunk_sums(qip_prec prec, const void *psi, uint64_t len, uint
   return cudaGetLastError();
 }
 
+// ---------------------------------------------------------------------------------
+// inverse-CDF sampling (qipb200_state_sample; decision rules in sample.cuh)
+// ---------------------------------------------------------------------------------
+static const int kScanThreads = 1024;
+
+// Inclusive scan over the warp; the same additions in the same order as sample_warp_scan.
+__device__ __forceinline__ double warp_incl_scan(double v) {
+  const int lane = threadIdx.x & 31;
+  for (int o = 1; o < 32; o <<= 1) {
+    const double x = __shfl_up_sync(0xffffffffu, v, o);
+    if (lane >= o) v = v + x;
+  }
+  return v;
+}
+
+// In-place inclusive scan of a[] in blocks of kScanThreads; block_tot[b] = total of block b (when non-NULL).
+__global__ void __launch_bounds__(kScanThreads) k_sample_scan(double *a, uint64_t n, double *block_tot) {
+  __shared__ double w[kScanThreads / 32];
+  const uint64_t i = (uint64_t)blockIdx.x * kScanThreads + threadIdx.x;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  double v = warp_incl_scan(i < n ? a[i] : 0.0);
+  if (lane == 31) w[warp] = v;
+  __syncthreads();
+  if (warp == 0) w[lane] = warp_incl_scan(w[lane]);
+  __syncthreads();
+  if (warp > 0) v += w[warp - 1];
+  if (i < n) a[i] = v;
+  if (block_tot && threadIdx.x == kScanThreads - 1) block_tot[blockIdx.x] = v;
+}
+
+// a[i] += prefix[b - 1] for every element of block b >= 1 (prefix = the scanned block totals).
+__global__ void __launch_bounds__(kScanThreads) k_sample_add(double *a, uint64_t n, const double *prefix) {
+  const uint64_t i = (uint64_t)(blockIdx.x + 1) * kScanThreads + threadIdx.x;
+  if (i < n) a[i] += prefix[blockIdx.x];
+}
+
+cudaError_t launch_sample_scan(double *d, uint64_t n, cudaStream_t s, uint64_t *launches) {
+  const uint64_t blocks = (n + kScanThreads - 1) / kScanThreads;
+  if (blocks <= 1) {
+    k_sample_scan<<<1, kScanThreads, 0, s>>>(d, n, nullptr);
+    ++*launches;
+    return cudaGetLastError();
+  }
+  double *tot = nullptr;
+  cudaError_t e = cudaMallocAsync((void **)&tot, blocks * sizeof(double), s);
+  if (e != cudaSuccess) return e;
+  k_sample_scan<<<(unsigned)blocks, kScanThreads, 0, s>>>(d, n, tot);
+  ++*launches;
+  e = cudaGetLastError();
+  if (e == cudaSuccess) e = launch_sample_scan(tot, blocks, s, launches);
+  if (e == cudaSuccess) {
+    k_sample_add<<<(unsigned)(blocks - 1), kScanThreads, 0, s>>>(d, n, tot);
+    ++*launches;
+    e = cudaGetLastError();
+  }
+  cudaError_t f = cudaFreeAsync(tot, s);
+  return e != cudaSuccess ? e : f;
+}
+
+// One warp per draw: owner rank, chunk search, scan of the chunk in 32-amplitude groups (sample.cuh).
+// out[j] = global index (as a double: < 2^53, exact) on the owner, 0 on every other rank.
+template <typename R>
+__global__ void __launch_bounds__(kThreads)
+    k_sample_resolve(const R *__restrict__ psi, const double *__restrict__ P, const double *__restrict__ totals,
+                     const double *__restrict__ draws, double *__restrict__ out, const SampleArgs a) {
+  const uint64_t j = ((uint64_t)blockIdx.x * kThreads + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (j >= a.n_draws) return;  // uniform over the warp
+  double t;
+  if (sample_owner(totals, a.world, draws[j], &t) != a.rank) {
+    if (lane == 0) out[j] = 0.0;
+    return;
+  }
+  uint64_t c = sample_chunk(P, a.chunks, t);
+  double base = c ? P[c - 1] : 0.0;
+  uint64_t last_nonzero = c << a.chunk_log2;
+  for (; c < a.chunks; ++c) {
+    const uint64_t begin = c << a.chunk_log2, end = begin + (1ull << a.chunk_log2);
+    for (uint64_t g = begin; g < end; g += 32) {
+      const uint64_t i = g + lane;
+      double p = 0.0;
+      if (i < end) {
+        const typename Vec2<R>::type v = *reinterpret_cast<const typename Vec2<R>::type *>(psi + 2 * i);
+        p = (double)v.x * (double)v.x + (double)v.y * (double)v.y;
+      }
+      const double incl = warp_incl_scan(p);
+      const unsigned hit = __ballot_sync(0xffffffffu, i < end && sample_crosses(base, incl, t));
+      if (hit) {
+        if (lane == 0) out[j] = (double)(a.index_base + g + (uint64_t)(__ffs(hit) - 1));
+        return;
+      }
+      const unsigned nz = __ballot_sync(0xffffffffu, p > 0.0);
+      if (nz) last_nonzero = g + (uint64_t)(31 - __clz(nz));
+      base += __shfl_sync(0xffffffffu, incl, 31);
+    }
+  }
+  if (lane == 0) out[j] = (double)(a.index_base + last_nonzero);
+}
+
+cudaError_t launch_sample_resolve(qip_prec prec, const void *psi, const double *P, const double *totals,
+                                  const double *draws, double *out, const SampleArgs &a, cudaStream_t s,
+                                  uint64_t *launches) {
+  const uint64_t warps_per_block = kThreads / 32;
+  const unsigned grid = (unsigned)((a.n_draws + warps_per_block - 1) / warps_per_block);
+  if (grid == 0) return cudaSuccess;
+  if (prec == QIP_F32)
+    k_sample_resolve<float><<<grid, kThreads, 0, s>>>((const float *)psi, P, totals, draws, out, a);
+  else
+    k_sample_resolve<double><<<grid, kThreads, 0, s>>>((const double *)psi, P, totals, draws, out, a);
+  ++*launches;
+  return cudaGetLastError();
+}
+
+struct OutcomeArgs {
+  uint64_t n_draws;
+  uint32_t n_bits;
+  uint8_t bitpos[64];
+};
+
+// res[j]: global index as a double -> outcome bits as a uint64, in place.
+__global__ void __launch_bounds__(kThreads) k_sample_outcomes(double *res, const __grid_constant__ OutcomeArgs a) {
+  const uint64_t j = (uint64_t)blockIdx.x * kThreads + threadIdx.x;
+  if (j >= a.n_draws) return;
+  const uint64_t index = (uint64_t)res[j];
+  reinterpret_cast<uint64_t *>(res)[j] = sample_outcome(index, a.bitpos, a.n_bits);
+}
+
+cudaError_t launch_sample_outcomes(double *res, uint64_t n_draws, const uint8_t *bitpos, uint32_t n_bits,
+                                   cudaStream_t s, uint64_t *launches) {
+  if (n_bits > 64) return cudaErrorInvalidValue;
+  if (n_draws == 0) return cudaSuccess;
+  OutcomeArgs a;
+  a.n_draws = n_draws;
+  a.n_bits = n_bits;
+  for (uint32_t j = 0; j < n_bits; ++j) a.bitpos[j] = bitpos[j];
+  k_sample_outcomes<<<grid_for(n_draws), kThreads, 0, s>>>(res, a);
+  ++*launches;
+  return cudaGetLastError();
+}
+
 template <typename R>
 __global__ void __launch_bounds__(kThreads)
     k_collapse(R *__restrict__ psi, uint64_t len, uint64_t index_base, uint64_t row_mask,

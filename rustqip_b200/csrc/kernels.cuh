@@ -6,6 +6,7 @@
 #include <cstdint>
 
 #include "opcompile.h"
+#include "sample.cuh"
 
 namespace qipb200 {
 
@@ -58,9 +59,26 @@ cudaError_t launch_set_basis(qip_prec prec, void *psi, uint64_t len, uint64_t in
 cudaError_t launch_measure_probs(qip_prec prec, const void *psi, uint64_t len, uint64_t index_base,
                                  const uint32_t *bitpos, uint32_t n_bits, double *d_hist, cudaStream_t s,
                                  uint64_t *launches);
-// per-chunk sums of |a|^2 (chunk = 2^chunk_log2 amplitudes) for inverse-CDF sampling.
+// per-chunk sums of |a|^2 (chunk = 2^chunk_log2 amplitudes): the one read sweep of inverse-CDF sampling.
 cudaError_t launch_chunk_sums(qip_prec prec, const void *psi, uint64_t len, uint32_t chunk_log2,
                               double *d_sums, cudaStream_t s, uint64_t *launches);
+// Inverse-CDF sampling (qipb200_state_sample; rules in sample.cuh).
+// d[0..n) <- its inclusive prefix sum, in a fixed order (repeated calls give identical bits).
+cudaError_t launch_sample_scan(double *d, uint64_t n, cudaStream_t s, uint64_t *launches);
+struct SampleArgs {
+  uint64_t n_draws;
+  uint64_t chunks;      // of this shard, 2^chunk_log2 amplitudes each
+  uint64_t index_base;  // global index of the shard's first amplitude
+  uint32_t chunk_log2;
+  int rank, world;      // totals[0..world) are the ranks' totals
+};
+// out[j] = global index drawn by draws[j] if this rank owns the draw, else 0 (P = inclusive prefix of the chunk sums).
+cudaError_t launch_sample_resolve(qip_prec prec, const void *psi, const double *P, const double *totals,
+                                  const double *draws, double *out, const SampleArgs &a, cudaStream_t s,
+                                  uint64_t *launches);
+// res[j] (a global index held as a double) <- its outcome bits as a uint64, bit i from bitpos[i].
+cudaError_t launch_sample_outcomes(double *res, uint64_t n_draws, const uint8_t *bitpos, uint32_t n_bits,
+                                   cudaStream_t s, uint64_t *launches);
 // measure_state: zero where (index & row_mask) != measured_mask, else scale by p_mult.
 cudaError_t launch_collapse(qip_prec prec, void *psi, uint64_t len, uint64_t index_base,
                             uint64_t row_mask, uint64_t measured_mask, double p_mult, cudaStream_t s,

@@ -223,6 +223,16 @@ class State:
         self._chk(_lib.lib().qipb200_state_soft_measure(self._h, _ptr(idx), len(idx), float(r), C.byref(m)))
         return int(m.value)
 
+    def sample(self, indices: Sequence[int], draws) -> np.ndarray:
+        """soft_measure for every draw in `draws` (floats in [0, 1]) from one read of the state; the state is unchanged.
+        Returns the outcomes as uint64, bit i from indices[i]."""
+        idx = np.ascontiguousarray(np.asarray(list(indices), dtype=np.uint64))
+        r = np.ascontiguousarray(np.asarray(draws, dtype=np.float64).reshape(-1))
+        out = np.empty(max(1, r.shape[0]), dtype=np.uint64)
+        self._chk(_lib.lib().qipb200_state_sample(self._h, _ptr(idx), len(idx), _ptr(r) if r.shape[0] else _ptr(out),
+                                                  r.shape[0], _ptr(out)))
+        return out[: r.shape[0]]
+
     def collapse(self, indices: Sequence[int], measured: int, prob: float):
         idx = np.ascontiguousarray(np.asarray(list(indices), dtype=np.uint64))
         self._chk(_lib.lib().qipb200_state_collapse(self._h, _ptr(idx), len(idx), int(measured), float(prob)))
